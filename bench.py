@@ -2,6 +2,7 @@
 """bench.py -- the measurement contract (one JSON line on stdout from rank 0).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload NAME] [--no-secondary]
+                    [--dump-outputs DIR]
 
 N > 1 is launched by the driver as
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
@@ -13,6 +14,12 @@ events), max over ranks, barrier + synchronize on both sides.
 The main line is BASELINE cfg 3 (benchmarks/workloads.py::InterleavedCfg3) through the reference surface
 ``MMInterleaved.forward``; the other BASELINE configurations that fit one GPU (cfg 2, cfg 4, cfg 5) are timed
 afterwards with the same procedure at a few steps each and attached as ``"secondary": {name: {...}}`` objects.
+
+``--dump-outputs DIR`` writes, after each workload's timed steps, what its last timed step (the last step of the
+end-to-end loop) computed as ``DIR/<workload>.<output>.npy`` (float32, or float64 for float64 and integer outputs; an
+output of more than 2**20
+elements is reduced to a fixed seeded sample of them).  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -28,10 +35,20 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def positive_int(text):
+    n = int(text)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {n}")
+    return n
+
+
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=positive_int, default=10, help="timed steps of the main workload")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="auto")
@@ -39,7 +56,24 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the cfg 2 / cfg 4 / cfg 5 secondary measurements")
     ap.add_argument("--secondary", default="", help="comma-separated subset of secondary workloads to run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write each workload's last timed step's outputs to DIR/<workload>.<output>.npy")
     return ap.parse_args()
+
+
+def dump_outputs(directory, workload, outputs, written):
+    """Write ``outputs`` ({name: tensor}) as float32 / float64 .npy files; returns ``written`` + their bytes."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach().cpu()
+        a = (t.double() if t.dtype == torch.float64 or not t.is_floating_point() else t.float()).numpy()
+        written += a.nbytes
+        if written > DUMP_LIMIT_BYTES:
+            raise SystemExit(f"--dump-outputs: more than {DUMP_LIMIT_BYTES} bytes at {workload}.{name}")
+        np.save(os.path.join(directory, f"{workload}.{name}.npy"), a)
+    return written
 
 
 class ClockSampler:
@@ -200,6 +234,9 @@ def main():
     wl = workloads.make(args.workload, rank=rank, world=world, local_batch=args.local_batch)
     wl.setup()
     line = measure(wl, args.steps, args.warmup, dist, rank, world, local_rank, cpu_baseline=not args.no_cpu_baseline)
+    dumped = 0
+    if args.dump_outputs and rank == 0:
+        dumped = dump_outputs(args.dump_outputs, wl.name, wl.outputs(), dumped)
     wl.teardown()
 
     main_name = workloads.AUTO if args.workload == "auto" else args.workload
@@ -212,6 +249,8 @@ def main():
                 sw.setup()
                 line["secondary"][name] = measure(sw, sw.default_steps, sw.default_warmup, dist, rank, world, local_rank,
                                                   cpu_baseline=False)
+                if args.dump_outputs and rank == 0:
+                    dumped = dump_outputs(args.dump_outputs, name, sw.outputs(), dumped)
                 sw.teardown()
             except Exception as e:          # a secondary must never take the main line down
                 import traceback

@@ -42,6 +42,18 @@ def ncu_traffic(kernel_key):
     return json.load(open(p)).get(kernel_key)
 
 
+OUTPUT_SAMPLE = 2 ** 20      # elements kept of an output larger than this (bench.py --dump-outputs)
+
+
+def output_sample(t, seed=0):
+    """``t`` itself, or OUTPUT_SAMPLE of its elements in flat order at fixed seeded positions when it is larger."""
+    n = t.numel()
+    if n <= OUTPUT_SAMPLE:
+        return t
+    idx = torch.randint(0, n, (OUTPUT_SAMPLE,), generator=torch.Generator().manual_seed(seed)).sort().values
+    return t.reshape(-1)[idx.to(t.device)]
+
+
 def msda_algorithmic_bytes(N, S, M, D, L, Lq, P, elem_size):
     """SURVEY.md 8d / BASELINE.md section 3: value + loc(2) + weight(1) + out, + shape tables."""
     return elem_size * (N * S * M * D + 3 * N * Lq * M * L * P + N * Lq * M * D) + 24 * L
@@ -170,6 +182,10 @@ class Workload:
         ms = [a.elapsed_time(b) for a, b in self._kernel_events]
         return {"launches": len(ms), "avg_ms": sum(ms) / len(ms) if ms else None}
 
+    def outputs(self):
+        """{name: tensor}: what the last timed step computed, as its caller receives it (bench.py --dump-outputs)."""
+        raise NotImplementedError
+
     def teardown(self):
         pass
 
@@ -278,6 +294,9 @@ class MsdaCfg3(Workload):
 
     def result_checksum(self):
         return self.last.float().sum().reshape(1).to("cuda")
+
+    def outputs(self):
+        return {"out": output_sample(self.last)}             # the step's last layer
 
     def h2d_bytes(self):
         return sum(t.numel() * t.element_size() for lay in self.layers_h for t in lay)
@@ -408,6 +427,7 @@ class InterleavedCfg3(Workload):
 
     def teardown(self):
         self._patch.restore()
+        self.last_logits = None
 
     def reset_counters(self):
         super().reset_counters()
@@ -426,7 +446,8 @@ class InterleavedCfg3(Workload):
         with torch.no_grad():
             out = self.model(text_ids=ids, image_tensors=images, num_image_per_seq=nimg, attention_mask=None,
                              max_num_image=self.N_IMG, return_loss=False)
-            return out["text_logits"].argmax(-1)
+            self.last_logits = out["text_logits"]
+            return self.last_logits.argmax(-1)
 
     def step_device(self):
         self.last = self._forward(self.dev_sets[self._i % self.N_SETS])
@@ -443,6 +464,9 @@ class InterleavedCfg3(Workload):
 
     def result_checksum(self):
         return self.last.sum().reshape(1).float()
+
+    def outputs(self):
+        return {"text_ids": self.last, "text_logits": output_sample(self.last_logits)}
 
     def h2d_bytes(self):
         return sum(t.numel() * t.element_size() for t in self.host)
@@ -665,6 +689,9 @@ class SdCfg4(Workload):
     def result_checksum(self):
         return self.last.float().sum().reshape(1)
 
+    def outputs(self):
+        return {"latents": output_sample(self.last)}
+
     def h2d_bytes(self):
         return sum(t.numel() * t.element_size() for t in self.host)
 
@@ -810,6 +837,9 @@ class GenerateCfg5(Workload):
 
     def result_checksum(self):
         return (self.last[0].sum().float() + self.last[1].float().sum()).reshape(1)
+
+    def outputs(self):
+        return {"text_ids": self.last[0], "image_latents": output_sample(self.last[1])}
 
     def h2d_bytes(self):
         return sum(t.numel() * t.element_size() for t in self.host)

@@ -2,6 +2,7 @@
 container (``/root/reference`` is absent on the GPU box, so the vectors travel instead).
 
     python tests/golden/make_golden.py            # writes tests/golden/*.npz
+    python tests/golden/make_golden.py ref_cuda   # on a B200 after build(): msda_ref_cuda_sampled.npz
 
 The reference ships no golden vectors for this path (SURVEY.md section 4: the pickle that
 ops/tests/compare_with_data.py:112-114 expects is not in the repository), so these fixtures
@@ -9,9 +10,14 @@ are outputs of the reference's own code run here:
 
   msda_core_*.npz   ms_deform_attn_core_pytorch (ops/functions/ms_deform_attn_func.py:47-67),
                     fp32 and fp64, on seeded inputs that are stored alongside the outputs
+  oracle_msda_loc_modes.npz, oracle_mmfs_seeded.npz, sincos_1d.npz, reference_layouts.npz
+                    ("reference_checks"): core / MMFS outputs, sin-cos tables and checkpoint layouts
+  msda_ref_cuda_sampled.npz
+                    ("ref_cuda"): the reference's own CUDA forward / backward (oracle/_ref/) on a B200
 """
 from __future__ import annotations
 
+import json
 import os
 import sys
 
@@ -538,9 +544,158 @@ def make_tokenizer(full=False):
     print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB")
 
 
+# ---------------------------------------------------------------------------------------------------------
+# Outputs of the reference that the tests used to compute from the reference tree (or from its CUDA op built into
+# oracle/_ref/) at test time.  Large outputs are kept as golden_sample(): a fixed, evenly strided subset.
+# ---------------------------------------------------------------------------------------------------------
+GOLDEN_SAMPLE = 1024
+
+
+def golden_sample(t, k=GOLDEN_SAMPLE):
+    """``k`` evenly strided elements of ``t`` in flat order (all of them if ``t`` is smaller)."""
+    flat = t.reshape(-1)
+    n = flat.numel()
+    return flat if n <= k else flat[torch.arange(k, dtype=torch.long) * n // k]
+
+
+# ms_deform_attn_core_pytorch on one shape under every location mode: (N, shapes, M, D, Lq, P); seed = mode index
+CORE_MODES_CASE = (2, [(12, 10), (6, 5), (3, 3)], 3, 16, 50, 5)
+CORE_MODES = ("uniform", "clustered", "edges")
+
+
+def make_core_modes(ref_ns):
+    core = ref_ns.func.ms_deform_attn_core_pytorch
+    N, shapes, M, D, Lq, P = CORE_MODES_CASE
+    arrays = {}
+    for seed, mode in enumerate(CORE_MODES):
+        v, s, st, loc, a = make_msda_inputs(N, shapes, M, D, Lq, P, seed=seed, loc_mode=mode)
+        arrays[f"{mode}_fp64"] = golden_sample(core(v.double(), s, loc.double(), a.double())).numpy()
+        arrays[f"{mode}_fp32"] = golden_sample(core(v, s, loc, a)).numpy()
+        arrays[f"{mode}_input_sha1"] = np.array(input_digest(v, loc, a))
+    path = os.path.join(HERE, "oracle_msda_loc_modes.npz")
+    np.savez_compressed(path, **arrays)
+    print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB")
+
+
+# the reference MMFS module on a second llm_tiny-shaped case with seeded weights (every branch non-zero)
+MMFS_SEEDED = dict(MMFS_CASES["llm_tiny"], seed=77, N=2, Lq=5)
+
+
+def mmfs_seeded_state_dict(template):
+    sd = seeded_state_dict(template, seed=7700)
+    sd["ignore_token"] = 0.3 * torch.randn(sd["ignore_token"].shape, generator=torch.Generator().manual_seed(7701))
+    return sd
+
+
+def make_mmfs_seeded(ref_ns):
+    case = MMFS_SEEDED
+    mod = ref_ns.mmfs.MMFS(**case["ctor"]).eval()
+    sd = mmfs_seeded_state_dict(mod.state_dict())
+    mod.load_state_dict(sd)
+    query, refpts, feat, ss, starts, mask = mmfs_case_inputs(case)
+    with torch.no_grad():
+        out = mod(query, refpts, feat, ss, starts, None, mask)
+    path = os.path.join(HERE, "oracle_mmfs_seeded.npz")
+    np.savez_compressed(path, out_fp32=out.numpy(), weight_checksum=np.array(float(sum(v.double().sum() for v in sd.values()))))
+    print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB")
+
+
+# utils/pos_embed.py get_1d_sincos_pos_embed_from_grid: (embed_dim, positions, rows kept, columns kept)
+SINCOS_CASES = ((16, 40, slice(None), slice(None)), (5120, 7, slice(None), slice(None, None, 13)),
+                (64, 2048, slice(None, None, 29), slice(None)))
+
+
+def make_sincos(ref_ns):
+    f = ref_ns.pos_embed.get_1d_sincos_pos_embed_from_grid
+    arrays = {f"d{dim}_n{n}": f(dim, np.arange(n, dtype=np.float32))[rows, cols] for dim, n, rows, cols in SINCOS_CASES}
+    path = os.path.join(HERE, "sincos_1d.npz")
+    np.savez_compressed(path, **arrays)
+    print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB")
+
+
+def ref_llama_config():
+    from transformers import LlamaConfig
+    extra = ("cross_attention_frequency", "spatial_shapes", "image_embed_dim")
+    cfg = LlamaConfig(**{k: v for k, v in LLAMA_TINY.items() if k not in extra}, hidden_act="silu")
+    for k in extra:
+        setattr(cfg, k, LLAMA_TINY[k])
+    return cfg
+
+
+def make_layouts(ref_ns):
+    """Checkpoint layouts (parameter / buffer names and shapes) of the reference LlamaModel (LLAMA_TINY) and MMFSNet
+    (MMFSNET_TINY): what a checkpoint saved from the reference holds."""
+    arrays = {}
+    for tag, mod in (("llama", ref_ns.llama.LlamaModel(ref_llama_config())), ("mmfsnet", ref_ns.sd_mmfs.MMFSNet(**MMFSNET_TINY))):
+        sd = mod.state_dict()
+        arrays[f"{tag}_keys"] = np.array(list(sd.keys()))
+        arrays[f"{tag}_shapes"] = np.array(json.dumps([list(v.shape) for v in sd.values()]))
+    path = os.path.join(HERE, "reference_layouts.npz")
+    np.savez_compressed(path, **arrays)
+    print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB")
+
+
+def load_layout(tag):
+    z = np.load(os.path.join(HERE, "reference_layouts.npz"))
+    return dict(zip([str(k) for k in z[f"{tag}_keys"]], json.loads(str(z[f"{tag}_shapes"]))))
+
+
+# the reference's own CUDA op (oracle/_ref/, built by oracle/build_ref.py) run on a B200: forward on the cases of
+# tests/test_msda_gpu.py::test_against_the_reference_cuda_op, backward on those of test_msda_bwd_gpu.py
+REF_CUDA_FWD_CASES, REF_CUDA_FWD_DTYPES = (0, 1, 2, 3, 5), ("float32", "float16", "float64")
+REF_CUDA_BWD_DTYPES = ("float32", "float16")
+
+
+def ref_cuda_fwd_inputs(case, dtype):
+    from tests.test_msda_gpu import CASES
+    N, shapes, M, D, Lq, P = CASES[case]
+    return make_msda_inputs(N, shapes, M, D, Lq, P, seed=300 + case, loc_mode="clustered", dtype=dtype)
+
+
+def ref_cuda_bwd_inputs(dtype):
+    from tests.test_msda_bwd_gpu import CASES
+    N, shapes, M, D, Lq, P = CASES[1]
+    v, s, st, loc, a = make_msda_inputs(N, shapes, M, D, Lq, P, seed=77, loc_mode="clustered", dtype=dtype)
+    go = torch.randn((N, Lq, M * D), generator=torch.Generator().manual_seed(2)).to(dtype)
+    return v, s, st, loc, a, go
+
+
+def make_ref_cuda():
+    from oracle import ref_cuda
+    ref = ref_cuda.load()
+    arrays = {}
+    for case in REF_CUDA_FWD_CASES:
+        for name in REF_CUDA_FWD_DTYPES:
+            dt = getattr(torch, name)
+            v, s, st, loc, a = ref_cuda_fwd_inputs(case, dt)
+            out = ref.ms_deform_attn_forward(v.to("cuda", dt), s.cuda(), st.cuda(), loc.to("cuda", dt), a.to("cuda", dt), 64)
+            arrays[f"fwd{case}_{name}"] = golden_sample(out.cpu()).numpy()
+            arrays[f"fwd{case}_{name}_input_sha1"] = np.array(input_digest(v.float(), loc.float(), a.float()))
+    for name in REF_CUDA_BWD_DTYPES:
+        dt = getattr(torch, name)
+        v, s, st, loc, a, go = ref_cuda_bwd_inputs(dt)
+        grads = ref.ms_deform_attn_backward(v.to("cuda", dt), s.cuda(), st.cuda(), loc.to("cuda", dt), a.to("cuda", dt),
+                                            go.cuda(), 64)
+        for g, gname in zip(grads, ("grad_value", "grad_loc", "grad_attn")):
+            arrays[f"bwd_{name}_{gname}"] = golden_sample(g.cpu()).numpy()
+            arrays[f"bwd_{name}_{gname}_absmax"] = np.array(float(g.float().abs().max()))
+        arrays[f"bwd_{name}_input_sha1"] = np.array(input_digest(v.float(), loc.float(), a.float()))
+    path = os.path.join(HERE, "msda_ref_cuda_sampled.npz")
+    np.savez_compressed(path, **arrays)
+    print(f"{path}: {os.path.getsize(path) / 1024:.0f} KiB")
+
+
 if __name__ == "__main__":
     torch.manual_seed(0)
-    which = sys.argv[1:] or ["msda", "mmfs", "llama", "mmfsnet", "adapter", "imgdec", "tokenizer"]
+    which = sys.argv[1:] or ["msda", "mmfs", "llama", "mmfsnet", "adapter", "imgdec", "tokenizer", "reference_checks"]
+    if "reference_checks" in which:
+        ns = ref_loader.load()
+        make_core_modes(ns)
+        make_mmfs_seeded(ns)
+        make_sincos(ns)
+        make_layouts(ns)
+    if "ref_cuda" in which:         # needs a GPU and oracle/_ref/
+        make_ref_cuda()
     if "tokenizer" in which:
         make_tokenizer()
     if "tokenizer_full" in which:

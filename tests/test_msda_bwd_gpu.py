@@ -1,5 +1,5 @@
 """GPU parity of the MSDA backward against (a) autograd through the CPU restatement of the reference's PyTorch core
-in fp64 and (b) the reference's OWN CUDA backward (oracle/_ref) on the same B200.
+in fp64 and (b) the reference's OWN CUDA backward (built by oracle/build_ref.py) run on a B200.
 Tolerance fp32: |err| <= 1e-4 * max|ref| per tensor (atomics: summation order differs); 16-bit: 2e-2 * max|ref|."""
 import pytest
 import torch
@@ -40,20 +40,23 @@ def test_backward_matches_autograd_of_the_core(case, mode, dtype):
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.float16])
 def test_backward_matches_the_reference_cuda_op(dtype):
-    from oracle import ref_cuda
-    if not ref_cuda.available():
-        pytest.skip("oracle/_ref not built")
-    ref = ref_cuda.load()
+    """Its gradients (a strided sample of each, with the max |gradient| of the whole tensor) are stored in
+    tests/golden/msda_ref_cuda_sampled.npz by make_golden.make_ref_cuda."""
+    import os
+
+    import numpy as np
+    from tests.golden.make_golden import golden_sample, input_digest, ref_cuda_bwd_inputs
     import mm_interleaved_b200 as m
-    N, shapes, M, D, Lq, P = CASES[1]
-    v, s, st, loc, a = make_msda_inputs(N, shapes, M, D, Lq, P, seed=77, loc_mode="clustered", dtype=dtype)
-    go = torch.randn((N, Lq, M * D), generator=torch.Generator().manual_seed(2)).to(dtype)
+    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "msda_ref_cuda_sampled.npz"))
+    key = f"bwd_{str(dtype).split('.')[-1]}"
+    v, s, st, loc, a, go = ref_cuda_bwd_inputs(dtype)
+    assert input_digest(v.float(), loc.float(), a.float()) == str(z[key + "_input_sha1"]), "inputs do not reproduce"
     args = [v.to(DEV, dtype), s.to(DEV), st.to(DEV), loc.to(DEV, dtype), a.to(DEV, dtype), go.to(DEV)]
-    want = ref.ms_deform_attn_backward(*args, 64)
     got = m.ms_deform_attn_backward(*args, 64)
     tol = 1e-4 if dtype == torch.float32 else 2e-2
-    for g, w in zip(got, want):
-        assert (g.float() - w.float()).abs().max() <= tol * w.float().abs().max() + 1e-7
+    for g, name in zip(got, ("grad_value", "grad_loc", "grad_attn")):
+        w, w_max = torch.from_numpy(z[f"{key}_{name}"]), float(z[f"{key}_{name}_absmax"])
+        assert (golden_sample(g.cpu()).float() - w.float()).abs().max() <= tol * w_max + 1e-7, name
 
 
 def test_deterministic_backward_is_bit_reproducible_and_matches_the_float_atomic_path():

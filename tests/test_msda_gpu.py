@@ -265,26 +265,27 @@ def test_dropin_module_and_autograd_wrapper():
     assert o3.dtype == torch.float16
 
 
-def _ref_op():
-    from oracle import ref_cuda
-    if not ref_cuda.available():
-        pytest.skip("oracle/_ref (the reference's own CUDA op) was not built")
-    return ref_cuda.load()
-
-
 @pytest.mark.parametrize("dtype", [torch.float32, torch.float16, torch.float64])
 @pytest.mark.parametrize("case", [0, 1, 2, 3, 5])
 def test_against_the_reference_cuda_op(case, dtype):
     """The reference's OWN kernel (ops/src/cuda/ms_deform_im2col_cuda.cuh, compiled unmodified for sm_100a by
-    oracle/build_ref.py) run on the same B200 on the same inputs."""
-    ref = _ref_op()
+    oracle/build_ref.py) run on a B200 on the same inputs; its outputs (a strided sample) are stored in
+    tests/golden/msda_ref_cuda_sampled.npz by make_golden.make_ref_cuda."""
+    import os
+
+    import numpy as np
+    from tests.golden.make_golden import golden_sample, input_digest, ref_cuda_fwd_inputs
     m = _mod()
+    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "msda_ref_cuda_sampled.npz"))
+    key = f"fwd{case}_{str(dtype).split('.')[-1]}"
     N, shapes, M, D, Lq, P = CASES[case]
-    v, s, st, loc, a = make_msda_inputs(N, shapes, M, D, Lq, P, seed=300 + case, loc_mode="clustered", dtype=dtype)
+    v, s, st, loc, a = ref_cuda_fwd_inputs(case, dtype)
+    assert input_digest(v.float(), loc.float(), a.float()) == str(z[key + "_input_sha1"]), "inputs do not reproduce"
     args = [v.to(DEV, dtype), s.to(DEV), st.to(DEV), loc.to(DEV, dtype), a.to(DEV, dtype)]
-    want = ref.ms_deform_attn_forward(*args, 64)
-    got = m.ms_deform_attn_forward(*args, 64)
+    out = m.ms_deform_attn_forward(*args, 64)
     torch.cuda.synchronize()
+    assert out.shape == (N, Lq, M * D)
+    got, want = golden_sample(out.cpu()), torch.from_numpy(z[key])
     assert got.shape == want.shape and got.dtype == want.dtype
     if dtype == torch.float64:
         assert (got - want).abs().max() <= 1e-12

@@ -1,11 +1,14 @@
 """CPU tests: pin the oracle (oracle/msda_ref.c, oracle.msda_core_pytorch) against the golden
-vectors generated from the reference's own code, and against the reference itself when the
-tree is present (build container only)."""
+vectors generated from the reference's own code."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
-from oracle import (error_metrics, make_msda_inputs, msda_core_pytorch, msda_forward_ref, ref_loader)
-from tests._golden import load_msda_case, msda_case_names
+from oracle import error_metrics, make_msda_inputs, msda_core_pytorch, msda_forward_ref
+from tests._golden import GOLDEN, load_msda_case, msda_case_names
+from tests.golden.make_golden import CORE_MODES, CORE_MODES_CASE, golden_sample, input_digest
 
 # fp32 accumulation-order noise between the scalar restatement and grid_sample
 F32_TOL = dict(max_abs=2e-6, max_rel=2e-5)
@@ -64,13 +67,16 @@ def test_empty_and_degenerate_shapes():
     assert torch.count_nonzero(out0) == 0
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree only exists in the build container")
 def test_against_live_reference_core():
-    ref = ref_loader.load()
-    for seed, mode in enumerate(["uniform", "clustered", "edges"]):
-        v, s, st, loc, a = make_msda_inputs(2, [(12, 10), (6, 5), (3, 3)], 3, 16, 50, 5, seed=seed, loc_mode=mode)
-        r = ref.func.ms_deform_attn_core_pytorch(v.double(), s, loc.double(), a.double())
-        o = msda_forward_ref(v, s, st, loc, a)
+    """The reference's ms_deform_attn_core_pytorch under every location mode; its outputs (a strided sample) are
+    stored in tests/golden/oracle_msda_loc_modes.npz by make_golden.make_core_modes."""
+    z = np.load(os.path.join(GOLDEN, "oracle_msda_loc_modes.npz"))
+    N, shapes, M, D, Lq, P = CORE_MODES_CASE
+    for seed, mode in enumerate(CORE_MODES):
+        v, s, st, loc, a = make_msda_inputs(N, shapes, M, D, Lq, P, seed=seed, loc_mode=mode)
+        assert input_digest(v, loc, a) == str(z[f"{mode}_input_sha1"]), f"inputs of mode '{mode}' do not reproduce"
+        r = torch.from_numpy(z[f"{mode}_fp64"])
+        o = golden_sample(msda_forward_ref(v, s, st, loc, a))
         m = error_metrics(o, r)
         assert m["max_abs"] < F32_TOL["max_abs"], (mode, m)
-        assert torch.equal(msda_core_pytorch(v, s, loc, a), ref.func.ms_deform_attn_core_pytorch(v, s, loc, a))
+        assert torch.equal(golden_sample(msda_core_pytorch(v, s, loc, a)), torch.from_numpy(z[f"{mode}_fp32"]))

@@ -1,83 +1,92 @@
 """The reference's ``replace_*()`` start-up mechanism (inference.py:10-24) pointed at the B200 classes: after
-``replace_*_b200()`` the REFERENCE's own ``LlamaModel`` / ``LlamaMMFSAttention`` / ``MMFSNet`` constructors build B200
-modules, and a state dict saved from the unpatched reference loads into them with ``strict=True``.  CPU-only
-(construction + state-dict load; compute needs the GPU).  Skipped where /root/reference is absent (the GPU box)."""
+``replace_*_b200()`` every reference module that holds one of the replaced classes holds the B200 class instead, and a
+state dict saved from the unpatched reference loads into the B200 modules with ``strict=True``.  CPU-only
+(construction + state-dict load; compute needs the GPU).  The reference modules are stood in for by empty modules
+under the same names, holding the same bindings; the reference checkpoint layouts come from
+tests/golden/reference_layouts.npz (make_golden.make_layouts)."""
 import sys
+import types
 
-import pytest
 import torch
 
-from oracle import ref_loader
+from tests.golden.make_golden import LLAMA_TINY, MMFSNET_TINY, load_layout
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present (GPU box)")
-
-
-def _ref_llama_config():
-    from transformers import LlamaConfig
-    from tests.golden.make_golden import LLAMA_TINY
-    extra = ("cross_attention_frequency", "spatial_shapes", "image_embed_dim")
-    cfg = LlamaConfig(**{k: v for k, v in LLAMA_TINY.items() if k not in extra}, hidden_act="silu")
-    for k in extra:
-        setattr(cfg, k, LLAMA_TINY[k])
-    return cfg
+_REF = "mm_interleaved.models"
+_LLAMA_CLASSES = ("LlamaRMSNorm", "LlamaMLP", "LlamaAttention", "LlamaMMFSAttention", "LlamaDecoderLayer")
 
 
-def test_replace_functions_rebind_the_reference_and_checkpoints_load():
+def _stand_in_reference(monkeypatch):
+    """Modules named like the reference's, each binding its own placeholder classes; the MMFS class is bound a second
+    time where the reference imports it (``from ..modules import MMFS`` in ops/modules/__init__.py and sd_mmfs.py)."""
+    def module(name, **attrs):
+        mod = types.ModuleType(f"{_REF}.{name}")
+        for k, v in attrs.items():
+            setattr(mod, k, v)
+        monkeypatch.setitem(sys.modules, mod.__name__, mod)
+        return mod
+
+    mmfs_cls = type("MMFS", (torch.nn.Module,), {})
+    return types.SimpleNamespace(
+        func=module("utils.ops.functions.ms_deform_attn_func", MSDA=types.ModuleType("MultiScaleDeformableAttention")),
+        mmfs=module("utils.ops.modules.mmfs", MMFS=mmfs_cls),
+        modules=module("utils.ops.modules", MMFS=mmfs_cls),
+        llama=module("decoders.modeling_llama_mmfs", **{n: type(n, (torch.nn.Module,), {}) for n in _LLAMA_CLASSES}),
+        sd_mmfs=module("decoders.sd_mmfs", MMFS=mmfs_cls, MMFSNet=type("MMFSNet", (torch.nn.Module,), {}),
+                       MMFSBlock=type("MMFSBlock", (torch.nn.Module,), {})))
+
+
+def _reference_checkpoint(tag):
+    return {k: torch.zeros(shape) for k, shape in load_layout(tag).items()}
+
+
+def test_replace_functions_rebind_the_reference_and_checkpoints_load(monkeypatch):
     import mm_interleaved_b200 as b200
     from mm_interleaved_b200 import patch
-    ns = ref_loader.load()
-    if ns.llama is None or ns.sd_mmfs is None:
-        pytest.skip("reference decoders do not import in this environment")
+    ns = _stand_in_reference(monkeypatch)
     ref_mmfs_cls, ref_layer_cls, ref_net_cls = ns.mmfs.MMFS, ns.llama.LlamaDecoderLayer, ns.sd_mmfs.MMFSNet
-    cfg = _ref_llama_config()
-    ref_sd = ns.llama.LlamaModel(cfg).state_dict()                       # unpatched reference: the checkpoint layout
-    from tests.golden.make_golden import MMFSNET_TINY
-    ref_net_sd = ref_net_cls(**MMFSNET_TINY).state_dict()
+    ref_msda = ns.func.MSDA
     try:
         b200.replace_mmfs_b200()
-        assert ns.mmfs.MMFS is b200.MMFS and ns.sd_mmfs.MMFS is b200.MMFS   # (the llama file imports it lazily, :325)
-        assert sys.modules["mm_interleaved.models.utils.ops.modules"].MMFS is b200.MMFS
+        assert ns.mmfs.MMFS is b200.MMFS and ns.sd_mmfs.MMFS is b200.MMFS and ns.modules.MMFS is b200.MMFS
         assert sys.modules["MultiScaleDeformableAttention"].ms_deform_attn_forward is b200.ms_deform_attn_forward
         assert ns.func.MSDA is sys.modules["MultiScaleDeformableAttention"]
-        # reference LlamaMMFSAttention (still the reference class) now builds the B200 MMFS inside
-        xattn = ns.llama.LlamaMMFSAttention(cfg, layer_idx=0)
-        assert type(xattn.attn) is b200.MMFS and type(xattn).__module__.startswith("mm_interleaved.")
-        xattn.load_state_dict({k[len("layers.0.llama_cross_attn."):]: v for k, v in ref_sd.items()
-                               if k.startswith("layers.0.llama_cross_attn.")}, strict=True)
 
         b200.replace_llama_b200()
-        for name in ("LlamaRMSNorm", "LlamaMLP", "LlamaAttention", "LlamaMMFSAttention", "LlamaDecoderLayer"):
+        for name in _LLAMA_CLASSES:
             assert getattr(ns.llama, name) is getattr(b200, name)
-        model = ns.llama.LlamaModel(cfg)                                  # the reference's own LlamaModel glue
-        assert type(model).__module__.startswith("mm_interleaved.")
-        assert all(type(l) is b200.LlamaDecoderLayer for l in model.layers)
-        assert type(model.layers[0].llama_cross_attn.attn) is b200.MMFS and type(model.norm) is b200.LlamaRMSNorm
-        missing, unexpected = model.load_state_dict(ref_sd, strict=True)
-        assert not missing and not unexpected
-        assert set(model.state_dict().keys()) == set(ref_sd.keys())
 
         b200.replace_visual_b200()
         assert ns.sd_mmfs.MMFSNet is b200.MMFSNet and ns.sd_mmfs.MMFSBlock is b200.MMFSBlock
-        net = ns.sd_mmfs.MMFSNet(**MMFSNET_TINY)
-        net.load_state_dict(ref_net_sd, strict=True)
 
         b200.replace_all_b200()                                           # idempotent
-        assert ns.llama.LlamaDecoderLayer is b200.LlamaDecoderLayer
+        assert ns.llama.LlamaDecoderLayer is b200.LlamaDecoderLayer and ns.mmfs.MMFS is b200.MMFS
     finally:
         patch.restore_reference()
     assert ns.mmfs.MMFS is ref_mmfs_cls and ns.sd_mmfs.MMFS is ref_mmfs_cls and ns.llama.LlamaDecoderLayer is ref_layer_cls
-    assert ns.sd_mmfs.MMFSNet is ref_net_cls
+    assert ns.sd_mmfs.MMFSNet is ref_net_cls and ns.func.MSDA is ref_msda
+    assert "MultiScaleDeformableAttention" not in sys.modules or \
+        not getattr(sys.modules["MultiScaleDeformableAttention"], "_b200_dropin", False)
+
+    # checkpoints saved from the unpatched reference load into the B200 modules unchanged
+    model = b200.LlamaModel(b200.LlamaMMFSConfig(**LLAMA_TINY))
+    assert all(type(l) is b200.LlamaDecoderLayer for l in model.layers)
+    assert type(model.layers[0].llama_cross_attn.attn) is b200.MMFS and type(model.norm) is b200.LlamaRMSNorm
+    ref_sd = _reference_checkpoint("llama")
+    missing, unexpected = model.load_state_dict(ref_sd, strict=True)
+    assert not missing and not unexpected
+    assert set(model.state_dict().keys()) == set(ref_sd.keys())
+    xattn = model.layers[0].llama_cross_attn
+    xattn.load_state_dict({k[len("layers.0.llama_cross_attn."):]: v for k, v in ref_sd.items()
+                           if k.startswith("layers.0.llama_cross_attn.")}, strict=True)
+    b200.MMFSNet(**MMFSNET_TINY).load_state_dict(_reference_checkpoint("mmfsnet"), strict=True)
 
 
 def test_b200_top_level_model_keeps_the_reference_state_dict_layout():
     """``MMInterleaved`` (B200) exposes the reference's parameter names for the parts whose reference classes import
     here (decoder + text head + glue): every key of the reference ``LlamaModel`` / ``TextDecoder`` layout exists."""
+    import pytest
     import mm_interleaved_b200 as b200
-    from tests.golden.make_golden import LLAMA_TINY
-    ns = ref_loader.load()
-    if ns.llama is None:
-        pytest.skip("reference decoder does not import")
-    ref_keys = {"mm_decoder." + k for k in ns.llama.LlamaModel(_ref_llama_config()).state_dict().keys()}
+    ref_keys = {"mm_decoder." + k for k in load_layout("llama")}
     tiny_vt = dict(clip_config=b200.visual_tokenizer.CLIPVisionConfigLite(hidden_size=64, intermediate_size=128,
                                                                         num_hidden_layers=4, num_attention_heads=4,
                                                                         image_size=32, patch_size=8),
